@@ -30,6 +30,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -90,10 +91,10 @@ def _gen_stream(args):
 
 def frame_pool(name: str):
     """pool_streams synthetic sequences of pool_frames pairs + the frame-to-frame rotations in both
-    directions, cached under /tmp (generation is numpy, one process per sequence)."""
+    directions, cached in the temporary directory (generation is numpy, one process per sequence)."""
     cfg = CONFIGS[name]
     PS, NF = cfg["pool_streams"], cfg["pool_frames"]
-    cache = "/tmp/kvfe_bench_pool_v2_%s_%d_%d.npz" % (name, PS, NF)
+    cache = os.path.join(tempfile.gettempdir(), "kvfe_bench_pool_v2_%s_%d_%d.npz" % (name, PS, NF))
     if os.path.exists(cache):
         try:
             z = np.load(cache)
@@ -296,6 +297,75 @@ def run_reference(args):
 
 
 # ------------------------------------------------------------------------------------------------
+DUMP_SEED = 0
+DUMP_PACKET_BYTES = 24 << 20          # budget of the sampled packets' per-keypoint arrays
+DUMP_RECT_BYTES = 32 << 20            # budget of the sampled keyframes' rectified pairs (float32)
+
+
+def dump_plan(pass_count: int, B: int, cap: int, W: int, H: int):
+    """Which outputs of the last timed step --dump-outputs writes in full: a seeded sample of (pass, stream)
+    slots sized so that the whole dump stays under 64 MB (at most 38 float64 values per keypoint slot)."""
+    n = max(1, min(256, pass_count * B, DUMP_PACKET_BYTES // (38 * 8 * max(cap, 1))))
+    flat = np.sort(np.random.default_rng(DUMP_SEED).choice(pass_count * B, size=n, replace=False))
+    return {"want": {(int(f) // B, int(f) % B) for f in flat}, "n_rect": min(8, DUMP_RECT_BYTES // (2 * 4 * W * H)),
+            "got": {}}
+
+
+def dump_outputs(d: str, chk, kf, nkp, plan):
+    """Writes what the caller of kvfe_pipeline_* received in the last timed step as DIR/<name>.npy:
+    step_*        (passes, streams) per output: keyframe flag, keypoint count, output checksum (two 32-bit halves);
+    packet_*      the sampled packets (slots in packet_pass_stream): header values one row per packet, keypoint
+                  arrays concatenated in slot order (row counts: packet_n, packet_n_smart, packet_n_mesh_triangles);
+    rect_*        the rectified pairs of the first sampled keyframes (slots in rect_pass_stream).
+    Arrays with no elements are not written: the bench runs with the 2D mesh off, so no mesh triangles.
+    Every value written is finite: a non-finite entry (uR of a smart stereo measurement whose right keypoint is not
+    valid is NaN) is stored as 0 and marked in <name>_nonfinite (0 finite, 1 NaN, 2 +inf, 3 -inf), which is written
+    only for arrays holding such entries."""
+    from kimera_vio_b200.lib import PACKET_FIELDS
+    os.makedirs(d, exist_ok=True)
+
+    def save(name, a):
+        a = np.asarray(a)
+        if a.size == 0:
+            return
+        a = a if a.dtype == np.float32 else a.astype(np.float64)
+        bad = ~np.isfinite(a)
+        if bad.any():
+            code = np.where(np.isnan(a), 1, np.where(a > 0, 2, 3)) * bad
+            np.save(os.path.join(d, name + "_nonfinite.npy"), code.astype(np.float32))
+            a = np.where(bad, 0, a).astype(a.dtype)
+        np.save(os.path.join(d, name + ".npy"), a)
+
+    chk = chk.astype(np.uint64)
+    save("step_is_keyframe", kf.astype(np.float32))
+    save("step_n_keypoints", nkp.astype(np.float32))
+    save("step_checksum_hi", chk >> np.uint64(32))
+    save("step_checksum_lo", chk & np.uint64(0xFFFFFFFF))
+    keys = sorted(plan["got"])
+    pk = [plan["got"][k] for k in keys]
+    save("packet_pass_stream", np.array(keys).reshape(-1, 2))
+    per_kp = {name for name, _, _ in PACKET_FIELDS}
+    for name in pk[0]:
+        if name in ("left_rect", "right_rect", "stream", "tag"):
+            continue
+        vals = [p[name] for p in pk]
+        if name == "checksum":
+            v = np.array(vals, np.uint64)
+            save("packet_checksum_hi", v >> np.uint64(32))
+            save("packet_checksum_lo", v & np.uint64(0xFFFFFFFF))
+        elif name == "timestamp":
+            save("packet_timestamp_from_t0", np.array(vals, np.int64) - T0_NS)
+        elif name in per_kp:
+            save("packet_" + name, np.concatenate(vals))
+        else:
+            save("packet_" + name, np.stack([np.asarray(v) for v in vals]))
+    rk = [k for k in keys if "left_rect" in plan["got"][k]][:plan["n_rect"]]
+    save("rect_pass_stream", np.array(rk, np.int64).reshape(-1, 2))
+    for side in ("left_rect", "right_rect"):
+        if rk:
+            save("rect_" + side.split("_")[0], np.stack([plan["got"][k][side] for k in rk]).astype(np.float32))
+
+
 def run_gpu(args):
     name = args.config
     cfg = CONFIGS[name]
@@ -357,9 +427,10 @@ def run_gpu(args):
     OUTS = (kl.PipelineOutput * 1024)()
     outs_np = np.frombuffer(OUTS, dtype=out_dt)
 
-    def run(pl, keep_packets=0):
+    def run(pl, keep_packets=0, dump=None):
         """Pushes a whole plan (queue-ahead) and pops until everything is done.  Returns per-(pass, slot)
-        arrays of checksum / is_keyframe / n_keypoints (+ parsed packets of slot 0 for the first passes)."""
+        arrays of checksum / is_keyframe / n_keypoints (+ parsed packets of slot 0 for the first passes).
+        dump: dump_plan() of the plan's last step, whose sampled packets are parsed into dump["got"]."""
         n, streams, lp, rp, ts, Rm, tags = pl
         t_first = int(tags[0])
         chk = np.zeros((n // B, B), np.uint64)
@@ -381,6 +452,11 @@ def run_gpu(args):
             if keep_packets:
                 for i in np.nonzero((o["stream"] == 0) & (o["tag"] < keep_packets))[0]:
                     kept[int(o["tag"][i])] = pipe.parse(OUTS[int(i)], copy_rect=False)
+            if dump is not None:
+                for i in np.nonzero(o["tag"] >= dump["from"])[0]:
+                    key = (int(o["tag"][i]) - dump["from"], int(o["stream"][i]))
+                    if key in dump["want"]:
+                        dump["got"][key] = pipe.parse(OUTS[int(i)], copy_rect=dump["n_rect"] > 0)
             lib.kvfe_pipeline_release(ph, OUTS, m)
             done += m
         return chk, kf, nkp, kept
@@ -391,6 +467,10 @@ def run_gpu(args):
         torch.cuda.synchronize()
 
     N_PAR = 24            # passes of slot 0 compared with the oracle (parity self-check)
+    dump = None
+    if args.dump_outputs and rank == 0:       # sampled in the e2e run, the last timed one
+        dump = dump_plan(R_in, B, pipe.cap, W, H)
+        dump["from"] = n_pass - R_in
     res = {}
     for label, bl, br in (("value", dL.data_ptr(), dR.data_ptr()), ("e2e", pL.data_ptr(), pR.data_ptr())):
         pipe.reset()
@@ -403,7 +483,7 @@ def run_gpu(args):
         with sampler:
             ev0.record()
             t0 = time.perf_counter()
-            timed = run(pl)
+            timed = run(pl, dump=dump if label == "e2e" else None)
             ev1.record()
             barrier()
             wall = time.perf_counter() - t0
@@ -415,6 +495,9 @@ def run_gpu(args):
     # the two runs process the same frames: every output (packet + rectified images) must be byte-identical
     same_outputs = bool(np.array_equal(res["value"]["timed"][0], res["e2e"]["timed"][0]) and
                         np.array_equal(res["value"]["warm"][0], res["e2e"]["warm"][0]))
+    if dump is not None:
+        chk, kf, nkp, _ = res["e2e"]["timed"]
+        dump_outputs(args.dump_outputs, chk[-R_in:], kf[-R_in:], nkp[-R_in:], dump)
     kf_all = np.concatenate([res["e2e"]["warm"][1], res["e2e"]["timed"][1]])
     rho = float(res["e2e"]["timed"][1].mean())
     n_kp_mean = float(res["e2e"]["timed"][2].mean())
@@ -584,7 +667,12 @@ def main():
     ap.add_argument("--impl", default="kvfe", choices=["kvfe", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-pin", action="store_true", help="do not pin the rank to the GPU's NUMA node")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step delivered (step-wide flags and checksums, a seeded sample of "
+                         "packets and keyframe rectified pairs) as DIR/<name>.npy, float32/float64, under 64 MB")
     args = ap.parse_args()
+    if args.steps < 1 or args.inner < 1:
+        ap.error("--steps and --inner must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":

@@ -7,8 +7,9 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
-REF = "/root/reference"
-REF_DATA = os.path.join(REF, "tests", "data")
+# Kimera-VIO's shipped rig files and test fixtures, stored by tests/golden/make_reference_fixtures.py
+REF = os.path.join(ROOT, "tests", "golden", "reference")
+REF_DATA = os.path.join(REF, "data")
 
 
 def pytest_configure(config):
@@ -28,7 +29,3 @@ def pytest_collection_modifyitems(config, items):
     for item in items:
         if "gpu" in item.keywords:
             item.add_marker(skip)
-
-
-needs_reference = pytest.mark.skipif(not os.path.isdir(REF_DATA),
-                                     reason="/root/reference fixtures not present (GPU box)")

@@ -8,14 +8,13 @@ import torch
 import torch.distributed as dist
 import torch.multiprocessing as mp
 
-from conftest import REF, ROOT, needs_reference
+from conftest import REF, ROOT
 from kimera_vio_b200 import dist as kd
 from kimera_vio_b200.params import CameraParams, FrontendParams
 from kimera_vio_b200.rig import StereoRigSetup
 from kimera_vio_b200.synth import SynthStream
 
 
-@needs_reference
 def test_euroc_yaml_equals_inlined_defaults():
     p = FrontendParams.from_yaml(os.path.join(REF, "params/Euroc/FrontendParams.yaml"))
     q = FrontendParams.euroc()
@@ -31,7 +30,6 @@ def test_euroc_yaml_equals_inlined_defaults():
     assert l.distortion == CameraParams.euroc_left().distortion
 
 
-@needs_reference
 @pytest.mark.parametrize("rig", ["Euroc", "uHumans2", "D455", "KinectAzure", "EurocMono", "RealSenseIR", "Kitti"])
 def test_all_shipped_rigs_parse(rig):
     path = os.path.join(REF, "params", rig, "FrontendParams.yaml")
@@ -288,7 +286,6 @@ def test_should_be_keyframe_host_logic():
     assert 50 < n_true < 700
 
 
-@needs_reference
 def test_camera_yaml_distortion_models_and_depth_blocks():
     """CameraParams.from_yaml on the shipped camera files: distortion model names (CameraParams.cpp:114-140) and the RGB-D
     block (CameraParams.cpp:342-349)."""

@@ -1,8 +1,8 @@
 """Pin the oracle against the reference's own known-answer tests (SURVEY.md section 8(c)).
 
-Each test cites the reference test it replays (paths relative to /root/reference).  They need the
-reference fixtures, so they skip on the GPU box; the committed golden vectors in tests/golden/ are
-produced by the oracle pinned here.
+Each test cites the reference test it replays (paths relative to a Kimera-VIO checkout).  They read
+the reference's fixtures stored under tests/golden/reference (PNG images as lossless WebP); the
+committed golden vectors in tests/golden/ are produced by the oracle pinned here.
 """
 import os
 
@@ -10,12 +10,10 @@ import cv2
 import numpy as np
 import pytest
 
-from conftest import REF_DATA, needs_reference
+from conftest import REF_DATA
 from kimera_vio_b200.params import CameraParams, FrontendParams
 from oracle import frontend as ofe
 from oracle.rig import StereoRig
-
-pytestmark = needs_reference
 
 
 def _frame(img_rel):
@@ -36,7 +34,7 @@ def _bins(fr, p):
 # tests/testFeatureDetector.cpp:26-52
 def test_detector_no_nms_393():
     p = FrontendParams.from_yaml(os.path.join(REF_DATA, "ForFeatureDetector/frontendParams-noNMS.yaml"))
-    f = _frame("ForStereoFrame/left_fisheye_img_0.png")
+    f = _frame("ForStereoFrame/left_fisheye_img_0.webp")
     ofe.FeatureDetector(p).feature_detection(f, None)
     assert len(f.keypoints) == 393
 
@@ -45,7 +43,7 @@ def test_detector_no_nms_393():
 def test_detector_no_nms_400():
     p = FrontendParams.from_yaml(os.path.join(REF_DATA, "ForFeatureDetector/frontendParams-noNMS.yaml"))
     p.quality_level = 1e-10
-    f = _frame("ForStereoFrame/left_fisheye_img_0.png")
+    f = _frame("ForStereoFrame/left_fisheye_img_0.webp")
     ofe.FeatureDetector(p).feature_detection(f, None)
     assert len(f.keypoints) == 400
 
@@ -53,7 +51,7 @@ def test_detector_no_nms_400():
 # tests/testFeatureDetector.cpp:83-106
 def test_detector_topn_300():
     p = FrontendParams.from_yaml(os.path.join(REF_DATA, "ForFeatureDetector/frontendParams-NMS-TopN.yaml"))
-    f = _frame("ForStereoFrame/left_fisheye_img_0.png")
+    f = _frame("ForStereoFrame/left_fisheye_img_0.webp")
     ofe.FeatureDetector(p).feature_detection(f, None)
     assert len(f.keypoints) == 300
 
@@ -61,7 +59,7 @@ def test_detector_topn_300():
 # tests/testFeatureDetector.cpp:109-150
 def test_detector_binning_20():
     p = FrontendParams.from_yaml(os.path.join(REF_DATA, "ForFeatureDetector/frontendParams-NMS-Binning.yaml"))
-    f = _frame("ForStereoFrame/left_fisheye_img_0.png")
+    f = _frame("ForStereoFrame/left_fisheye_img_0.webp")
     ofe.FeatureDetector(p).feature_detection(f, None)
     assert len(f.keypoints) == 20
     assert np.all(_bins(f, p) == 1)
@@ -73,7 +71,7 @@ def test_detector_binning_200():
     p.max_features_per_frame = 200
     p.quality_level = 1e-10
     p.enable_subpixel_corner_refinement = False
-    f = _frame("ForStereoFrame/left_fisheye_img_0.png")
+    f = _frame("ForStereoFrame/left_fisheye_img_0.webp")
     ofe.FeatureDetector(p).feature_detection(f, None)
     assert len(f.keypoints) == 200
     assert np.all(_bins(f, p) == 10)
@@ -84,7 +82,7 @@ def test_detector_binning_mask_140():
     p = FrontendParams.from_yaml(os.path.join(REF_DATA, "ForFeatureDetector/frontendParams-NMS-Binning2.yaml"))
     p.quality_level = 1e-10
     p.enable_subpixel_corner_refinement = False
-    f = _frame("ForStereoFrame/left_fisheye_img_0.png")
+    f = _frame("ForStereoFrame/left_fisheye_img_0.webp")
     ofe.FeatureDetector(p).feature_detection(f, None)
     assert len(f.keypoints) == 140
     cnt = _bins(f, p)
@@ -108,7 +106,7 @@ def test_stereo_matcher_shifted_849_of_900():
     assert abs(rig.baseline - 0.110078) < 1e-4            # tests/testStereoMatcher.cpp:148
     p = FrontendParams()                                  # struct defaults, as in the fixture
     m = ofe.StereoMatcher(p, rig)
-    img = cv2.imread(os.path.join(d, "left_img_0.png"), cv2.IMREAD_GRAYSCALE)
+    img = cv2.imread(os.path.join(d, "left_img_0.webp"), cv2.IMREAD_GRAYSCALE)
     corners = cv2.goodFeaturesToTrack(img, 100, 0.01, 10, blockSize=3, useHarrisDetector=False, k=0.04)
     corners = corners.reshape(-1, 2)
     count_valid = total = 0
@@ -150,8 +148,8 @@ def test_process_first_frame_35_corners():
     p.max_point_dist = 500
     p.templ_cols = 9
     p.subpixel_refinement_stereo = True
-    imgl = cv2.imread(os.path.join(d, "img_distort_left.png"), cv2.IMREAD_GRAYSCALE)
-    imgr = cv2.imread(os.path.join(d, "img_distort_right.png"), cv2.IMREAD_GRAYSCALE)
+    imgl = cv2.imread(os.path.join(d, "img_distort_left.webp"), cv2.IMREAD_GRAYSCALE)
+    imgr = cv2.imread(os.path.join(d, "img_distort_right.webp"), cv2.IMREAD_GRAYSCALE)
 
     def load(path):
         vals = open(path).read().split()
@@ -258,14 +256,13 @@ def test_rotational_flow_predictor_reference_numbers():
         assert abs(float(x) - ex) <= 1e-1 and abs(float(y) - ey) <= 1e-1, ((x, y), (ex, ey))
 
 
-@needs_reference
 def test_mesher_create_mesh_2d_reference_fixture():
     """tests/testMesher.cpp:147-197: the four corners of chessboard_small.png (UtilsOpenCV::ExtractCorners =
     goodFeaturesToTrack(100, 0.01, 10, blockSize 3)) give two triangles, vertices in the order
     (kp2, kp1, kp3) and (kp1, kp2, kp0); no keypoints -> no triangle."""
     import cv2
     from oracle import mesher
-    img = cv2.imread(os.path.join(REF_DATA, "chessboard_small.png"), cv2.IMREAD_GRAYSCALE)
+    img = cv2.imread(os.path.join(REF_DATA, "chessboard_small.webp"), cv2.IMREAD_GRAYSCALE)
     kps = cv2.goodFeaturesToTrack(img, 100, 0.01, 10, None, None, 3, False, 0.04).reshape(-1, 2)
     assert len(kps) == 4
     size = (img.shape[1], img.shape[0])
