@@ -266,12 +266,20 @@ extern "C" int kvfe_create(const kvfe_config* cfg, const kvfe_rig* rig, kvfe_ctx
   dc.min_distance = c.min_distance; dc.nms_enabled = c.enable_non_max_suppression; dc.nms_type = c.non_max_suppression_type;
   dc.hbins = c.nr_horizontal_bins; dc.vbins = c.nr_vertical_bins; dc.n_active_bins = 0;
   for (int i = 0; i < 64; ++i) { dc.bin_mask[i] = i < nbins ? c.binning_mask[i] : 0; if (i < nbins && c.binning_mask[i]) dc.n_active_bins++; }
-  dc.quality = (float)c.quality_level;   // GFTTDetector stores a double; the product is formed in double
+  dc.quality = c.quality_level;          // GFTTDetector keeps a double: maxVal * qualityLevel in double, rounded to float once
   dc.subpix_enabled = c.enable_subpixel_corner_refinement; dc.subpix_win = c.subpix_window_size;
   dc.subpix_iters = std::min(std::max(c.subpix_max_iters, 1), 100); dc.subpix_zero = c.subpix_zero_zone;
   { double e = std::max(c.subpix_epsilon, 0.); dc.subpix_eps2 = e * e; }
   dc.sobel_tail_start = c.sobel_cpu_tail_start;
-  { size_t want = (size_t)dc.W * dc.H / 8; size_t p = 8192; while (p < want) p <<= 1; dc.cand_cap = (int)p; }
+  // every interior pixel can be a candidate (a flat plateau of the response passes the 3x3 max test), and
+  // cv::goodFeaturesToTrack keeps them all; a power of two because the min_distance < 1 path sorts the list
+  // in place, padded to the next power of two
+  {
+    size_t want = (size_t)(dc.W - 2) * (dc.H - 2), p = 8192;
+    while (p < want) p <<= 1;
+    if (p > ((size_t)1 << 30)) { delete ctx; return set_err(nullptr, KVFE_ERR_INVALID_ARG, "image too large for the corner candidate list"); }
+    dc.cand_cap = (int)p;
+  }
   // rectified calibration: Cal3_S2Stereo from P1 (StereoCamera.cpp:75-82)
   dc.fx = rig->P1[0]; dc.fy = rig->P1[5]; dc.cxr = rig->P1[2]; dc.cyr = rig->P1[6]; dc.baseline = rig->baseline;
   // stereo stripe geometry (StereoMatcher.cpp:214-231)

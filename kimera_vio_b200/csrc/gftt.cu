@@ -407,7 +407,7 @@ __global__ void __launch_bounds__(256) cand_kernel(DevCfg dc, DevBuf db, int mod
   const float* e = db.eig + (size_t)b * W * H;
   float maxv = ord2f(db.eig_max[b]);
   if (!(maxv > -INFINITY)) maxv = 0.f;              // empty mask: minMaxLoc leaves maxVal = 0
-  const float thr = (float)((double)maxv * (double)dc.quality);
+  const float thr = (float)((double)maxv * dc.quality);   // cv::threshold(eig, eig, maxVal * qualityLevel, ...)
   for (int k = 0; k < 8; ++k) {
     const int y = blockIdx.y * 64 + k * 8 + (threadIdx.x >> 5);
     if (x < 1 || y < 1 || x > W - 2 || y > H - 2) continue;

@@ -110,7 +110,7 @@ struct DevCfg {          // passed by value to kernels
   // detector
   int max_features, max_before_anms, min_distance, nms_enabled, nms_type;
   int hbins, vbins; unsigned char bin_mask[64]; int n_active_bins;
-  float quality;
+  double quality;        // quality_level as given: cv::GFTTDetector keeps it a double
   int subpix_enabled, subpix_win, subpix_iters, subpix_zero; double subpix_eps2;
   int sobel_tail_start;
   int cand_cap;          // candidate list capacity per stream

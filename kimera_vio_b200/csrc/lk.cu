@@ -126,24 +126,31 @@ __global__ void __launch_bounds__(LK_WARPS * 32) lk_kernel(DevCfg dc, DevBuf db,
     }
     __syncwarp();
     // Structure tensor with OpenCV's SIMD128 accumulation order (pinned against cv2: scratch probe,
-    // 2400/2400 points bit-exact): four float lanes, pixel i (row-major) -> lane i % 4, sequential
-    // float accumulation per lane, final (L0 + L2) + (L1 + L3).  Lanes 0..11 = 3 sums x 4 chains.
+    // 2400/2400 points bit-exact): within each window row, pixels x < win & ~3 go to four float lanes
+    // (x -> lane x % 4, sequential float accumulation per lane over the rows), the rest of the row to a
+    // scalar float sum; final tail + ((L0 + L2) + (L1 + L3)).  Lanes 0..11 = 3 sums x 4 chains, lanes
+    // 12..14 the three tails (zero when win is a multiple of 4).
     float A11, A12, A22;
     {
       float acc = 0.f;
-      const int q = lane >> 2, c = lane & 3;
-      if (lane < 12) {
+      const int nv = win & ~3;
+      if (lane < 15) {
+        const int q = lane < 12 ? lane >> 2 : lane - 12, c = lane & 3;
         const short* u = (q == 2) ? s.Iy : s.Ix;
         const short* v = (q == 0) ? s.Ix : s.Iy;
-        for (int i = c; i < win * win; i += 4) acc = acc + (float)((int)u[i] * (int)v[i]);
+        for (int y = 0; y < win; ++y) {
+          const int r = y * win;
+          if (lane < 12) { for (int x = c; x < nv; x += 4) acc = acc + (float)((int)u[r + x] * (int)v[r + x]); }
+          else { for (int x = nv; x < win; ++x) acc = acc + (float)((int)u[r + x] * (int)v[r + x]); }
+        }
       }
       float l2 = __shfl_down_sync(KVFE_FULL_MASK, acc, 2);
       float l1 = __shfl_down_sync(KVFE_FULL_MASK, acc, 1);
       float l3 = __shfl_down_sync(KVFE_FULL_MASK, acc, 3);
       float tot = (acc + l2) + (l1 + l3);          // valid in lanes 0, 4, 8
-      A11 = __shfl_sync(KVFE_FULL_MASK, tot, 0) * FLT_SCALE;
-      A12 = __shfl_sync(KVFE_FULL_MASK, tot, 4) * FLT_SCALE;
-      A22 = __shfl_sync(KVFE_FULL_MASK, tot, 8) * FLT_SCALE;
+      A11 = (__shfl_sync(KVFE_FULL_MASK, acc, 12) + __shfl_sync(KVFE_FULL_MASK, tot, 0)) * FLT_SCALE;
+      A12 = (__shfl_sync(KVFE_FULL_MASK, acc, 13) + __shfl_sync(KVFE_FULL_MASK, tot, 4)) * FLT_SCALE;
+      A22 = (__shfl_sync(KVFE_FULL_MASK, acc, 14) + __shfl_sync(KVFE_FULL_MASK, tot, 8)) * FLT_SCALE;
     }
     float D = A11 * A22 - A12 * A12;
     float minEig = (A22 + A11 - sqrtf((A11 - A22) * (A11 - A22) + 4.f * A12 * A12)) / (float)(2 * win * win);
@@ -179,24 +186,33 @@ __global__ void __launch_bounds__(LK_WARPS * 32) lk_kernel(DevCfg dc, DevBuf db,
         diffv[i] = (short)(descale(p[0] * iw00 + p[1] * iw01 + p[jw] * iw10 + p[jw + 1] * iw11, 14 - 5) - s.I[i]);
       }
       __syncwarp();
-      // OpenCV's SIMD128 order for the mismatch vector (pinned against cv2): groups of 8 pixels
-      // (row-major); chain m in 0..3 accumulates float(int32(d[k]*G[k] + d[k+4]*G[k+4])), k = 8g + m;
-      // final (c0 + c2) + (c1 + c3).  Lanes 0..7 = 2 sums x 4 chains.
+      // OpenCV's SIMD128 order for the mismatch vector (pinned against cv2): within each window row, groups
+      // of 8 pixels x < win & ~7; chain m in 0..3 accumulates float(int32(d[k]*G[k] + d[k+4]*G[k+4])),
+      // k = 8g + m; the rest of the row goes to a scalar float sum; final tail + ((c0 + c2) + (c1 + c3)).
+      // Lanes 0..7 = 2 sums x 4 chains, lanes 8..9 the two tails (zero when win is a multiple of 8).
       float b1, b2;
       {
         float acc = 0.f;
-        if (lane < 8) {
-          const short* G = (lane < 4) ? s.Ix : s.Iy;
+        const int nv = win & ~7;
+        if (lane < 10) {
+          const short* G = (lane < 4 || lane == 8) ? s.Ix : s.Iy;
           const int m = lane & 3;
-          for (int k = m; k + 4 < win * win; k += 8)
-            acc = acc + (float)((int)diffv[k] * (int)G[k] + (int)diffv[k + 4] * (int)G[k + 4]);
+          for (int y = 0; y < win; ++y) {
+            const int r = y * win;
+            if (lane < 8) {
+              for (int k = r + m; k < r + nv; k += 8)
+                acc = acc + (float)((int)diffv[k] * (int)G[k] + (int)diffv[k + 4] * (int)G[k + 4]);
+            } else {
+              for (int k = r + nv; k < r + win; ++k) acc = acc + (float)((int)diffv[k] * (int)G[k]);
+            }
+          }
         }
         float l2 = __shfl_down_sync(KVFE_FULL_MASK, acc, 2);
         float l1 = __shfl_down_sync(KVFE_FULL_MASK, acc, 1);
         float l3 = __shfl_down_sync(KVFE_FULL_MASK, acc, 3);
         float tot = (acc + l2) + (l1 + l3);        // valid in lanes 0 and 4
-        b1 = __shfl_sync(KVFE_FULL_MASK, tot, 0) * FLT_SCALE;
-        b2 = __shfl_sync(KVFE_FULL_MASK, tot, 4) * FLT_SCALE;
+        b1 = (__shfl_sync(KVFE_FULL_MASK, acc, 8) + __shfl_sync(KVFE_FULL_MASK, tot, 0)) * FLT_SCALE;
+        b2 = (__shfl_sync(KVFE_FULL_MASK, acc, 9) + __shfl_sync(KVFE_FULL_MASK, tot, 4)) * FLT_SCALE;
       }
       __syncwarp();
       float dxv = (float)((A12 * b2 - A22 * b1) * D);
