@@ -87,7 +87,9 @@ struct StepIO {
   int force_kf;                  // Frame::isKeyframe_ of this frame (user-enforced keyframe, VisionImuFrontend.cpp:209)
   const unsigned char* next_srcL;   // images of the stream's NEXT frame when it is already queued (dense rows, 16-byte
   const unsigned char* next_srcR;   // aligned), else null: pulled into the staging slot while this step computes
-  unsigned long long pad1[6];
+  const unsigned char* srcD;     // RGB-D: the frame's depth image (device or mapped host memory), srcD_pitch bytes per row
+  unsigned long long srcD_pitch;
+  unsigned long long pad1[4];
   volatile unsigned long long done_seq;   // device -> host, own 64-byte line
   unsigned long long pad2[7];
   volatile unsigned long long decided_seq;  // split step graphs: published right after the keyframe decision, own line
@@ -128,6 +130,13 @@ struct DevCfg {          // passed by value to kernels
   // mesher
   int mesh_on; float subdiv_factor;
   int mono;              // frontend_type 1: MonoVisionImuFrontend (no stereo half)
+  // frontend_type 2: RgbdVisionImuFrontend -- the depth image of stream b at DevBuf::depth + b * depth_stride, depth_row bytes
+  // per row (W * 2 or W * 4); kvfe_depth_params as the kernels use them
+  int rgbd, depth_type;
+  size_t depth_row, depth_stride;
+  float depth_to_m, depth_min;                  // getDepthAtPoint
+  float depth_lo, depth_hi; unsigned int depth_lo16, depth_hi16;   // getDetectionMask bounds (f32 / u16 images)
+  double depth_fx_b;                            // fx * virtual_baseline (RgbdFrame.cpp:66)
   // ingest
   int equalize;          // cv::equalizeHist on both raw images before anything else (stereo_matching_params.equalize_image)
 };
@@ -139,6 +148,7 @@ struct DevBuf {
   unsigned char* rectL;        // B * img_stride
   unsigned char* rectR;
   unsigned char* mask;         // B * img_stride (u8 0/255)
+  unsigned char* depth;        // RGB-D: B * depth_stride (null otherwise)
   float* eig;                  // B * W*H
   unsigned int* eig_max;       // B (ordered-int encoded float)
   unsigned long long* cand;    // B * cand_cap  (float bits << 32 | pixel index)
@@ -282,6 +292,7 @@ int launch_prep(const DevCfg& dc, const DevBuf& db, const CamModel* d_cam, const
                 const double* Rin, const StepIO* io, cudaStream_t s);
 int launch_fetch_io(const DevCfg& dc, const DevBuf& db, const StepIO* io, int cur_slot, cudaStream_t s);
 int launch_fetch_right_io(const DevCfg& dc, const DevBuf& db, const StepIO* io, int cur_slot, int mode_mask, cudaStream_t s);
+int launch_fetch_depth_io(const DevCfg& dc, const DevBuf& db, const StepIO* io, int mode_mask, cudaStream_t s);
 int launch_prefetch_io(const DevCfg& dc, const DevBuf& db, const StepIO* io, int cur_slot, unsigned int* counter, cudaStream_t s);
 int launch_publish_io(const DevCfg& dc, const DevBuf& db, StepIO* io, unsigned int* counter, cudaStream_t s);
 int launch_track_pre(const DevCfg& dc, const DevBuf& db, cudaStream_t s);
@@ -303,6 +314,9 @@ int launch_rgbd_fill(const DevCfg& dc, const CamModel* d_cam, const unsigned cha
                      float depth_to_meters, float min_depth, double fx_b, const float* kp_x, const float* kp_y, const int* left_status,
                      const float* left_x, const float* left_y, const double* versors, int n, int* right_status, float* right_x,
                      float* right_y, double* depth_out, double* p3d, float* right_kp_x, float* right_kp_y, cudaStream_t s);
+// the same two on frame slot k of every stream whose mode is in mode_mask (frame-level RGB-D step)
+int launch_depth_mask_batch(const DevCfg& dc, const DevBuf& db, int mode_mask, cudaStream_t s);
+int launch_rgbd_fill_batch(const DevCfg& dc, const DevBuf& db, const CamModel* d_cam, int mode_mask, cudaStream_t s);
 // mesh.cu
 bool mesh_fits_smem(const DevCfg& dc);
 size_t mesh_global_ws_ints(const DevCfg& dc);

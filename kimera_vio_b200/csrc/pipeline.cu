@@ -27,6 +27,7 @@ namespace {
 
 struct PipeIn {
   const unsigned char* L; const unsigned char* R; size_t pitch;
+  const unsigned char* D; size_t dpitch;       // RGB-D: depth image (null otherwise)
   long long ts; double Rm[9]; unsigned long long tag;
   int force_kf;
 };
@@ -41,6 +42,7 @@ struct PipeStream {
   std::vector<PipeOutSlot> out;
   unsigned char* out_block = nullptr; // one pinned allocation behind `out`
   unsigned char* stage[2] = {nullptr, nullptr};   // pinned staging of pageable inputs, per I/O slot (lazy)
+  unsigned char* dstage[2] = {nullptr, nullptr};  // the same for a pageable depth image (RGB-D)
   bool force_next = false;            // kvfe_pipeline_force_keyframe: Frame::isKeyframe_ of the next pushed frame (under mu)
   // dispatcher-private
   std::deque<PipeFlight> fl;
@@ -70,9 +72,18 @@ struct kvfe_pipeline {
   std::atomic<int> failed{0};
   std::mutex err_mu; char err[512] = "";
   bool split = false;                 // split step graphs (keyframe kernels launched only for keyframes)
+  bool rgbd = false;                  // frontend_type 2: frames come with a depth image (kvfe_pipeline_push_rgbd)
+  size_t depth_row = 0;               // bytes per depth row (W * 2 or W * 4)
 };
 
 static thread_local char g_pipe_create_err[512] = "";
+
+// KVFE_ERR_INVALID_ARG with a message, without marking the pipeline failed (nothing was enqueued)
+static int pipe_refuse(kvfe_pipeline* p, const char* msg) {
+  std::lock_guard<std::mutex> g(p->err_mu);
+  snprintf(p->err, sizeof(p->err), "%s", msg);
+  return KVFE_ERR_INVALID_ARG;
+}
 
 static int pipe_fail(kvfe_pipeline* p, int code, const char* msg) {
   if (p) {
@@ -227,6 +238,27 @@ static const unsigned char* resolve_src(kvfe_pipeline* p, PipeStream* s, int io_
   return d;
 }
 
+// the same for a depth image (RGB-D): in place when the SMs can read it, else staged densely through a pinned slot
+static const unsigned char* resolve_depth(kvfe_pipeline* p, PipeStream* s, int io_slot, const unsigned char* ptr, size_t pitch,
+                                          size_t* out_pitch) {
+  cudaPointerAttributes a;
+  cudaError_t e = cudaPointerGetAttributes(&a, ptr);
+  if (e == cudaSuccess && (a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged)) { *out_pitch = pitch; return ptr; }
+  if (e == cudaSuccess && a.type == cudaMemoryTypeHost && a.devicePointer) {
+    *out_pitch = pitch;
+    return static_cast<const unsigned char*>(a.devicePointer);
+  }
+  if (e != cudaSuccess) cudaGetLastError();
+  const size_t rb = p->depth_row;
+  if (!s->dstage[io_slot] && cudaMallocHost((void**)&s->dstage[io_slot], rb * p->H) != cudaSuccess) return nullptr;
+  unsigned char* d = s->dstage[io_slot];
+  if (pitch == rb) memcpy(d, ptr, rb * p->H);
+  else for (int y = 0; y < p->H; ++y) memcpy(d + (size_t)y * rb, ptr + (size_t)y * pitch, rb);
+  p->n_staged.fetch_add(1, std::memory_order_relaxed);
+  *out_pitch = rb;
+  return d;
+}
+
 // device-visible address of a buffer the SMs can read in place (device memory, or pinned mapped host memory); null otherwise
 static const unsigned char* direct_src(const unsigned char* ptr) {
   cudaPointerAttributes a;
@@ -302,6 +334,13 @@ static void worker_main(kvfe_pipeline* p, int widx) {
         }
         if (!L || !R || pl != pr) { pipe_fail(p, KVFE_ERR_CUDA, "pipeline: cannot stage the input images"); break; }
         io->srcL = L; io->srcR = R; io->src_pitch = pl;
+        io->srcD = nullptr; io->srcD_pitch = 0;
+        if (p->rgbd) {
+          size_t pd = 0;
+          const unsigned char* D = resolve_depth(p, s, io_slot, in.D, in.dpitch, &pd);
+          if (!D) { pipe_fail(p, KVFE_ERR_CUDA, "pipeline: cannot stage the depth image"); break; }
+          io->srcD = D; io->srcD_pitch = pd;
+        }
         io->next_srcL = nullptr; io->next_srcR = nullptr;
         if (have_next) {
           const unsigned char* nl = direct_src(nxt.L);
@@ -365,6 +404,7 @@ extern "C" void kvfe_pipeline_destroy(kvfe_pipeline* p) {
     if (s->ctx) { cudaStreamSynchronize(s->ctx->stream); kvfe_destroy(s->ctx); }
     if (s->out_block) cudaFreeHost(s->out_block);
     for (int i = 0; i < 2; ++i) if (s->stage[i]) cudaFreeHost(s->stage[i]);
+    for (int i = 0; i < 2; ++i) if (s->dstage[i]) cudaFreeHost(s->dstage[i]);
     delete s;
   }
   delete p;
@@ -387,6 +427,12 @@ extern "C" int kvfe_pipeline_create(const kvfe_config* cfg, const kvfe_rig* rig,
   // 0.87): a step graph with a parallel branch costs twice the launch time on the host and the branches of 32
   // graphs compete for the 32 hardware work queues; the overlap across streams already hides the transfer
   p->pc.prefetch = pc->prefetch > 0 ? 1 : 0;
+  p->rgbd = cfg->frontend_type == 2;
+  if (p->rgbd) {
+    p->pc.prefetch = 0;            // the prefetch branch pulls the two 8-bit images of the next frame, not a depth image
+    p->pc.want_rectified = 0;      // no rectified pair: outputs carry null rect_left / rect_right
+    p->depth_row = (size_t)cfg->width * (cfg->depth.depth_type == KVFE_DEPTH_F32 ? 4 : 2);
+  }
   {
     // KVFE_PIPE_SPLIT=0/1 overrides (diagnostic); the prefetch branch lives in the single-graph variant only
     const char* e = getenv("KVFE_PIPE_SPLIT");
@@ -437,7 +483,7 @@ extern "C" int kvfe_pipeline_create(const kvfe_config* cfg, const kvfe_rig* rig,
       for (int k = 0; k < KVFE_PACKET_ARRAYS; ++k) p->pk_off[k] = s->ctx->db.pk_off[k];
     }
     const size_t pkb = (p->packet_bytes + 255) & ~(size_t)255, imb = (p->img + 255) & ~(size_t)255;
-    const size_t per = pkb + (pc->want_rectified ? 2 * imb : 0);
+    const size_t per = pkb + (p->pc.want_rectified ? 2 * imb : 0);
     if (cudaMallocHost((void**)&s->out_block, per * p->pc.output_slots) != cudaSuccess) {
       pipe_fail(nullptr, KVFE_ERR_CUDA, "pipeline: pinned output allocation failed");
       kvfe_pipeline_destroy(p);
@@ -446,7 +492,7 @@ extern "C" int kvfe_pipeline_create(const kvfe_config* cfg, const kvfe_rig* rig,
     memset(s->out_block, 0, per * p->pc.output_slots);
     for (int k = 0; k < p->pc.output_slots; ++k) {
       unsigned char* b = s->out_block + (size_t)k * per;
-      s->out.push_back(PipeOutSlot{b, pc->want_rectified ? b + pkb : nullptr, pc->want_rectified ? b + pkb + imb : nullptr});
+      s->out.push_back(PipeOutSlot{b, p->pc.want_rectified ? b + pkb : nullptr, p->pc.want_rectified ? b + pkb + imb : nullptr});
       s->free_out.push_back(k);
     }
   }
@@ -456,14 +502,20 @@ extern "C" int kvfe_pipeline_create(const kvfe_config* cfg, const kvfe_rig* rig,
 }
 
 static int push_one(kvfe_pipeline* p, int stream, const uint8_t* left, const uint8_t* right, size_t pitch,
-                    int64_t timestamp, const double* R, uint64_t tag, bool notify) {
+                    int64_t timestamp, const double* R, uint64_t tag, bool notify, const void* depth = nullptr,
+                    size_t depth_pitch = 0) {
   if (p && !right && !p->streams.empty() && p->streams[0]->ctx->dc.mono) right = left;      // mono front-end: no right camera
   if (!p || !left || !right || !R) return KVFE_ERR_INVALID_ARG;
+  if (p->rgbd != (depth != nullptr))        // wrong entry point for the front-end: refused, the pipeline stays usable
+    return pipe_refuse(p, p->rgbd ? "push: an RGB-D pipeline (frontend_type 2) takes kvfe_pipeline_push_rgbd"
+                                                      : "push_rgbd: not an RGB-D pipeline (frontend_type 2)");
   if (stream < 0 || stream >= (int)p->streams.size() || pitch < (size_t)p->W) return pipe_fail(p, KVFE_ERR_INVALID_ARG, "push: bad stream or pitch");
+  if (depth && depth_pitch < p->depth_row) return pipe_refuse(p, "push_rgbd: depth pitch smaller than a row");
   if (int f = p->failed.load()) return f;
   PipeStream* s = p->streams[stream];
   PipeIn in;
   in.L = left; in.R = right; in.pitch = pitch; in.ts = timestamp; in.tag = tag; in.force_kf = 0;
+  in.D = static_cast<const unsigned char*>(depth); in.dpitch = depth_pitch;
   memcpy(in.Rm, R, sizeof(in.Rm));
   {
     std::lock_guard<std::mutex> g(s->mu);
@@ -480,6 +532,13 @@ static int push_one(kvfe_pipeline* p, int stream, const uint8_t* left, const uin
 extern "C" int kvfe_pipeline_push(kvfe_pipeline* p, int stream, const uint8_t* left, const uint8_t* right, size_t pitch,
                                   int64_t timestamp, const double* R, uint64_t tag) {
   return push_one(p, stream, left, right, pitch, timestamp, R, tag, true);
+}
+
+// RGB-D: the intensity image stands in for the (absent) right image, like the mono front-end's
+extern "C" int kvfe_pipeline_push_rgbd(kvfe_pipeline* p, int stream, const uint8_t* img, size_t pitch, const void* depth,
+                                       size_t depth_pitch_bytes, int64_t timestamp, const double* R, uint64_t tag) {
+  if (!p || !img || !depth || !R) return KVFE_ERR_INVALID_ARG;
+  return push_one(p, stream, img, img, pitch, timestamp, R, tag, true, depth, depth_pitch_bytes);
 }
 
 extern "C" int kvfe_pipeline_push_many(kvfe_pipeline* p, int n, const int32_t* streams, const uint8_t* const* left,
